@@ -23,7 +23,13 @@ A second timed leg runs BASELINE configs[3], the one HBM-bound kernel of the pat
 `roofline_hbm`).  The queueing kernels are FP64-pipe bound (SURVEY 0.4): `roofline` reports the dominant kernel (the
 sizer) against the HBM peak as the contract asks — meaningless by construction — and against the measured FP64 peak.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--steps K sets the number of timed steps of every leg (resident step, end-to-end call, saturation kernel).
+--dump-outputs DIR writes, after the timed steps, what the last step of each timed leg computed as DIR/<name>.npy
+(float32 stays float32, everything else becomes float64): the candidates, the limited solution, the replica grid
+(frontier and per-level arrays) and the saturation outputs.  An output of more than 2^18 entries is written as the same
+seeded sample of its entries on every run, so two builds can be compared array by array.
 """
 from __future__ import annotations
 
@@ -37,6 +43,8 @@ import threading
 import time
 
 import numpy as np
+
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is cached next to the sources
 
 # Rank 0 prints ONE JSON line on stdout.  Libraries (NCCL's version banner, torchrun notices) write to file descriptor 1
 # too, so the descriptor is pointed at stderr for the whole run and the line goes out through a saved copy of it.
@@ -59,6 +67,8 @@ ALG_BYTES_PER_EVAL = 17.9                 # SURVEY.md 8(d): 16 B written + amort
 ALG_BYTES_PER_PAIR = 24 + 36.0 / A + 37   # sizing: 24 B + 36 B/A in, 37 B out per (server, accelerator)
 FP64_OPS_PER_STATE = 9.0                  # 5 FP64-pipe ops per pass-1 state, 13 per pass-2 state (DESIGN.md 4)
 METRIC = "(model,variant,replica) evals/sec"
+DUMP_SAMPLE = 1 << 18                     # --dump-outputs: entries kept of a larger output
+DUMP_BYTES = 64 << 20                     # --dump-outputs: size cap of all written arrays together
 
 
 def workload(scale: float = 1.0):
@@ -138,6 +148,50 @@ class ClockSampler(threading.Thread):
                 continue
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": smax or None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+# ---- --dump-outputs ---------------------------------------------------------------------------------------------------
+def _pick(n, seed):
+    """sorted indices into an output of n entries: all of them, or the same seeded sample of DUMP_SAMPLE draws"""
+    if n <= DUMP_SAMPLE:
+        return np.arange(n)
+    return np.unique(np.random.default_rng(seed).integers(0, n, DUMP_SAMPLE))
+
+
+def step_outputs(eng, R):
+    """What the last resident step left for its caller: the candidates and the limited solution of the whole system,
+    the replica grid of this rank's block of servers (frontier + per-level arrays, fetched one array at a time)."""
+    out = {}
+    cand = eng.candidates()
+    pick = _pick(cand["state"].size, 1)
+    out.update({"candidates_" + k: v.reshape(-1)[pick] for k, v in cand.items() if k != "n_solves"})   # a work count
+    sol = eng.solution()
+    pick = _pick(sol["state"].size, 4)
+    out.update({"solution_" + k: v if k.startswith("type_") else v[pick] for k, v in sol.items()})
+    front = eng.grid_fetch_frontier().reshape(-1)
+    out["grid_frontier"] = front[_pick(front.size, 2)]
+    n = front.size * R
+    pick = _pick(n, 3)
+    for i, (k, dt) in enumerate((("ok", np.uint8), ("ttft", np.float32), ("itl", np.float32), ("rho", np.float32),
+                                 ("tput", np.float32))):
+        buf = np.empty(max(n, 1), dt)
+        ptrs = [None] * 6
+        ptrs[i] = buf.ctypes.data
+        eng._check(eng.lib.wva_grid_fetch(eng.ctx, *ptrs), "wva_grid_fetch")
+        out["grid_" + k] = buf[pick]
+        del buf
+    return out
+
+
+def write_outputs(path, arrays):
+    arrays = {k: np.asarray(v, np.float32 if np.asarray(v).dtype == np.float32 else np.float64)
+              for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES} byte cap")
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 # ---- the reference algorithm on the host cores ------------------------------------------------------------------------
@@ -237,7 +291,12 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0, help="shrink the system (development only; 1.0 = configs[2])")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-saturation", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
@@ -344,13 +403,14 @@ def main():
         dist.all_reduce(cnt)
     ph = dict(zip(keys, ph.tolist()))
     size_solves, size_states, grid_solves, grid_states = cnt.tolist()
+    dump = step_outputs(eng, R) if args.dump_outputs and rank == 0 else None    # before the e2e arm replaces the grid
 
     # ---- end-to-end arm ---------------------------------------------------------------------------------------------------
     for _ in range(2):
         e2e_step()
     barrier()
     e0.record()
-    e2e_steps = max(2, args.steps // 2)
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         sol, fr = e2e_step()
     e1.record()
@@ -384,13 +444,17 @@ def main():
             eng.saturation_run(False)
         ks, xs = [], []
         barrier()
-        for _ in range(max(args.steps, 5)):
+        for _ in range(args.steps):
             flush.zero_()
             torch.cuda.synchronize()      # the flush runs on torch's stream, the kernel on the library's: no overlap
             eng.saturation_run(False)
             t = eng.timing()
             ks.append(t["saturation_ms"]); xs.append(t["exchange_ms"])
-        res = eng.saturation_fetch(fields=("partials", "partials_all"))
+        res = eng.saturation_fetch(fields=("partials", "partials_all") + (("var_target", "mod_flags") if dump is not None else ()))
+        if dump is not None:
+            dump["saturation_partials_all"] = res["partials_all"]
+            for k in ("var_target", "mod_flags"):
+                dump["saturation_" + k] = res[k][_pick(res[k].size, 5)]
         alg_loc = batch["n_replicas"] * 16 + batch["n_variants"] * 32 + M_loc * 40      # SURVEY 8(d)
         v = torch.tensor([float(np.mean(ks)), float(np.min(ks)), float(np.mean(xs))], dtype=torch.float64, device=dev)
         tot = torch.tensor([float(alg_loc), float(batch["n_replicas"])], dtype=torch.float64, device=dev)
@@ -471,6 +535,8 @@ def main():
             line["cpu_baseline"] = {k: v for k, v in cpu_reference_leg(args.ref_seconds).items()
                                     if k in ("value", "unit", "cores", "kind", "sample", "one_thread", "affinity_cpus",
                                              "cgroup_cpu_quota")}
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         emit(line)
     eng.close()
     if world > 1:
